@@ -1,4 +1,4 @@
-"""Drives the UNMODIFIED reference (baseline/_ref, staged by baseline/install_ref.py) through its own public control
+"""Drives the UNMODIFIED reference (oracle/_ref, staged by oracle/install_ref.py) through its own public control
 path — options -> models.create_model -> model.setup -> model.set_input -> model.optimize_parameters()
 (train.py:183-199, 268-282; models/base_model.py:1302-1377) — for bench.py's reference arm (CPU, all host threads) and
 for the GPU incumbent (the same stock code on cuda:0: fp32, and TF32 as train.py --with_tf32 sets it, :536-538).
@@ -17,7 +17,7 @@ import time
 from unittest import mock
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_ROOT = os.path.join(HERE, "_ref")
+REF_ROOT = os.path.join(os.path.dirname(HERE), "oracle", "_ref")
 
 OPTIONAL = [
     "thop", "torchviz", "piq", "lpips", "positional_encodings", "clip", "timm", "bitsandbytes", "imgaug",

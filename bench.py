@@ -1,6 +1,7 @@
 """bench.py — training-step throughput of the B200 path on BASELINE.json's configurations.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5]
+                    [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU, NCCL); rank 0 prints ONE JSON line.
 
@@ -20,10 +21,16 @@ UNetVid 8 x 128^2 (1 clip/GPU): same step definition through their trainers.
             `traffic` = DRAM read + write bytes of the implicit-GEMM launches of ONE step from the committed ncu launch
             list of the same step (profiles/r02_conv_traffic.json, config 2 only; null otherwise): DRAM bytes cannot be
             measured inside a timed run.
-  cpu_baseline / --impl reference: the UNMODIFIED reference (baseline/_ref, staged by baseline/install_ref.py) driven
+  cpu_baseline / --impl reference: the UNMODIFIED reference (oracle/_ref, staged by oracle/install_ref.py) driven
             through options -> create_model -> optimize_parameters() on the host cores (kind "reference"); the oracle
             port only if the staged reference is missing (kind "port").
   incumbent_gpu: the same unmodified reference on cuda:0 (cuDNN, fp32 and TF32), CUDA-event timed, reduced batch.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step handed its caller — DIR/loss.npy (the
+step's loss value(s), float64), DIR/params_<net>.npy (every trained network's updated weights, flattened in parameter
+order, float32) and DIR/ema.npy (the EMA copy, when the trainer keeps one) — 64 MB at most in all: an array over its
+share holds a fixed, seeded sample of its elements.  Weights and inputs are seeded, so two builds of the project can be
+compared output for output on the same arguments.
 """
 import argparse
 import contextlib
@@ -64,6 +71,8 @@ def parse():
     ap.add_argument("--no-incumbent", action="store_true")
     ap.add_argument("--cpu-steps", type=int, default=2)
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of CUDA-graph replay")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the last timed step's outputs to DIR/<name>.npy (64 MB at most)")
     a = ap.parse_args()
     info = CONFIG_INFO[a.config]
     a.batch = a.batch or info["batch"]
@@ -155,7 +164,7 @@ def cpu_threads():
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# reference arm / CPU baseline / GPU incumbent: the unmodified reference from baseline/_ref, in a child process
+# reference arm / CPU baseline / GPU incumbent: the unmodified reference from oracle/_ref, in a child process
 # ---------------------------------------------------------------------------------------------------------------------
 def _run_ref_runner(extra, timeout):
     env = dict(os.environ)
@@ -174,7 +183,7 @@ def _run_ref_runner(extra, timeout):
 
 
 def reference_available():
-    return os.path.exists(os.path.join(ROOT, "baseline", "_ref", "models", "base_model.py"))
+    return os.path.exists(os.path.join(ROOT, "oracle", "_ref", "models", "base_model.py"))
 
 
 def cpu_reference_throughput(size, steps, warmup=1, threads=None, budget_s=120.0):
@@ -193,14 +202,14 @@ def cpu_reference_throughput(size, steps, warmup=1, threads=None, budget_s=120.0
                                  res["s_per_step"])}
         note = "reference run failed (%s); oracle port instead" % err
     else:
-        note = "baseline/_ref missing; oracle port instead"
+        note = "oracle/_ref missing; oracle port instead"
     out = cpu_port_throughput(size, steps, threads, budget_s)
     out["note"] = note
     return out
 
 
 def cpu_port_throughput(size, steps, threads, budget_s):
-    """Fallback: the oracle's restatement of the same step (used only when baseline/_ref did not travel)."""
+    """Fallback: the oracle's restatement of the same step (used only when oracle/_ref did not travel)."""
     from oracle import palette_oracle as O
     torch.set_num_threads(threads)
     oc = O.OptimCfg(lr=1e-4)
@@ -234,7 +243,7 @@ def cpu_port_throughput(size, steps, threads, budget_s):
 def gpu_incumbent(size, batch=8, steps=3, warmup=3):
     """The unmodified reference on cuda:0 (its stock cuDNN path): strict fp32 and --with_tf32."""
     if not reference_available():
-        return {"unavailable": "baseline/_ref missing"}
+        return {"unavailable": "oracle/_ref missing"}
     out = {"batch": batch, "steps": steps, "warmup": warmup,
            "what": "unmodified reference (create_model -> optimize_parameters), cuDNN NCHW, cudnn.benchmark, "
                    "CUDA-event timed; batch %d (fp32 activations of batch 32 do not leave room beside this process)"
@@ -281,6 +290,7 @@ def build_workload(args, rank, world):
     """-> (trainer, host batch dict, images per step per GPU, workload string, algorithmic step FLOPs or None)"""
     from joligen_b200 import nets, synthetic
     from joligen_b200.trainer import PaletteTrainer
+    torch.manual_seed(1234)   # default initialisations and the in-step draws (noise, t): the same on every run
     h, w = args.size
     B = args.batch
     common = dict(in_channel=6, inner_channel=64, out_channel=3, tanh=False, n_timestep_train=2000,
@@ -364,6 +374,36 @@ def build_workload(args, rank, world):
     return tr, host, B, name, None
 
 
+DUMP_BYTES = 64 << 20
+
+
+def step_outputs(tr, out):
+    """What one training step hands its caller, on the host: the loss value(s) optimize_parameters() returned, the
+    updated weights of every network the trainer owns and its EMA copy.  An array over its share of DUMP_BYTES keeps a
+    fixed, seeded sample of its elements (the same positions for the same shapes)."""
+    losses = out if isinstance(out, (tuple, list)) else (out,)
+    arrays = {"loss": torch.stack([l.detach().double().reshape(()) for l in losses]).cpu()}
+    for name, m in sorted(vars(tr).items()):
+        if isinstance(m, torch.nn.Module) and any(True for _ in m.parameters()):
+            arrays["params_" + name] = torch.cat([p.detach().float().reshape(-1) for p in m.parameters()])
+    if isinstance(getattr(tr, "ema", None), torch.Tensor):
+        arrays["ema"] = tr.ema.detach().float().reshape(-1)
+    share = (DUMP_BYTES - 4096) // 4 // max(1, len(arrays) - 1)
+    for name, v in arrays.items():
+        if name != "loss" and v.numel() > share:
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:share].sort().values
+            v = v[idx.to(v.device)]
+        arrays[name] = v.cpu()
+    return arrays
+
+
+def dump_outputs(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), v.numpy())
+
+
 def ncu_conv_traffic(args):
     """DRAM bytes per step of the implicit-GEMM launches (ncu launch list committed under profiles/), config 2 at the
     default size only; None when there is no capture for the workload."""
@@ -413,12 +453,12 @@ def main():
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         ev0.record()
-        last = None
+        last = out = None
         for _ in range(steps):
             tr.set_input(host if from_host else dev)
-            loss = step_loss(tr.optimize_parameters())
+            out = tr.optimize_parameters()
             if from_host:
-                last = float(loss)  # D2H read of the step's loss
+                last = float(step_loss(out))  # D2H read of the step's loss
         ev1.record()
         barrier()
         ms = ev0.elapsed_time(ev1)
@@ -426,18 +466,20 @@ def main():
             t = torch.tensor([ms], device="cuda")
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t)
-        return ms / steps, last
+        return ms / steps, last, out
 
     run(max(args.warmup, 3), False)
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     L.launch_count[0] = 0
-    ms, _ = run(args.steps, False)
+    ms, _, out = run(args.steps, False)
     launches = L.launch_count[0]
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        outputs = step_outputs(tr, out)   # before the passes below train on
     run(1, True)
-    ms_e2e, last_loss = run(args.steps, True)
+    ms_e2e, last_loss, _ = run(args.steps, True)
 
     # instrumented pass: CUDA events around every C-ABI call; conv launches carry the FLOPs they issue
     recs = []
@@ -543,6 +585,8 @@ def main():
             if not args.no_incumbent:
                 line["incumbent_gpu"] = gpu_incumbent(args.size[0])
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()

@@ -1,15 +1,23 @@
-"""Import shim for running the UNMODIFIED reference (/root/reference) in the build container
+"""Import shim for running the UNMODIFIED reference (the copy build() staged under oracle/_ref, else the checkout)
 (TEST INFRASTRUCTURE — see oracle/__init__.py).  Optional third-party packages the reference
 imports at module level but never touches on the palette / unet_mha / resnet / NLayerD arithmetic
-path are replaced by MagicMock modules (SURVEY.md top table).  Used only by oracle/gen_golden.py;
-nothing on the GPU box reads /root/reference.
+path are replaced by MagicMock modules (SURVEY.md top table).  Used by the golden generators and by the tests
+that drive the reference's own training code.
 """
 import importlib.abc
 import importlib.machinery
+import os
 import sys
 from unittest import mock
 
-REFERENCE_ROOT = "/root/reference"
+_STAGED = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
+REFERENCE_ROOT = _STAGED if os.path.isdir(_STAGED) else os.environ.get("JG_REFERENCE_ROOT", "")
+
+
+def available():
+    """True where the reference's own code can run: the copy build() staged under oracle/_ref, or the checkout."""
+    return os.path.isfile(os.path.join(REFERENCE_ROOT, "models", "base_model.py"))
+
 
 MISSING = [
     "thop", "torchviz", "piq", "lpips", "positional_encodings", "clip", "timm", "bitsandbytes", "imgaug",

@@ -27,5 +27,5 @@ def test_reference_arm_prints_the_contract_line():
     assert "workload" in d["config"]
     assert d["cpu_baseline"]["cores"] == 2                       # the explicit thread count, not torchrun's 1
     assert d["steps"] == d["cpu_baseline"]["steps_timed"] == 1   # the line reports what was really timed
-    if os.path.exists(os.path.join(ROOT, "baseline", "_ref", "models", "base_model.py")):
+    if os.path.exists(os.path.join(ROOT, "oracle", "_ref", "models", "base_model.py")):
         assert d["cpu_baseline"]["kind"] == "reference"

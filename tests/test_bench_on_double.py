@@ -43,3 +43,26 @@ def test_graft_entry_smoke_runs_on_the_double():
         "import __graft_entry__ as g; g.smoke()"])
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode == 0 and "smoke ok" in r.stdout, (r.stdout[-500:], r.stderr[-2000:])
+
+
+def test_bench_dump_outputs_is_reproducible(tmp_path):
+    """--dump-outputs DIR: the last timed step's loss, updated weights and EMA copy as float32 / float64 .npy files,
+    64 MB at most in all, the same arrays from two runs with the same arguments, and other weights after one more timed
+    step (the dump is taken after the timed loop, whose length --steps sets)."""
+    import numpy as np
+    dumps = []
+    for run, steps in (("a", 2), ("b", 2), ("c", 3)):
+        out = tmp_path / run
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "bench_on_double.py"), "--config", "2", "--size",
+                            "32", "--batch", "2", "--steps", str(steps), "--warmup", "1", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=900, cwd=ROOT, env=dict(os.environ, OMP_NUM_THREADS="4"))
+        assert r.returncode == 0, r.stderr[-3000:]
+        assert json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])["steps"] == steps
+        dumps.append({p.name: np.load(p) for p in sorted(out.iterdir())})
+    a, b, c = dumps
+    assert {"loss.npy", "params_netG_A.npy", "ema.npy"} <= set(a) and set(a) == set(b)
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    for name, v in a.items():
+        assert v.dtype in (np.float32, np.float64) and np.isfinite(v).all(), name
+        assert np.array_equal(v, b[name]), name
+        assert not np.array_equal(v, c[name]), name

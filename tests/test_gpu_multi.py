@@ -126,7 +126,7 @@ def _worker(rank, world, port, out):
 
 def test_two_gpu_gradient_and_replicas():
     if not torch.cuda.is_available() or torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     import torch.multiprocessing as mp
     world = 2
     mgr = mp.Manager()

@@ -13,7 +13,10 @@ import torch
 
 import kernel_double as KD
 
-REF = "/root/reference"
+from oracle import ref_stubs  # noqa: E402
+
+REF_MISSING = "needs the reference's own code: build() stages it under oracle/_ref where the checkout is readable"
+
 
 
 def rel_l2(a, b):
@@ -115,7 +118,7 @@ def test_modulewise_dropin_signatures_nchw():
         assert ya.shape == (2, 16, 8, 8)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not ref_stubs.available(), reason=REF_MISSING)
 def test_reference_palette_model_trains_with_accelerated_generator(golden_dir):
     """THE drop-in claim: the UNMODIFIED reference's control path (options -> create_model -> setup -> set_input ->
     optimize_parameters(): compute_palette_loss, loss.backward(), AdamW, ema_step with its copy.deepcopy) with
@@ -234,58 +237,47 @@ def test_gan_nets_host_stack_vs_reference_golden(golden_dir):
         assert float((p.grad.double() - gref).norm()) <= 8e-2 * float(gref.norm()) + floor, k
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
-def test_accelerate_swaps_reference_gan_nets_and_matches_their_forward():
-    """accelerate() on the reference's own ResnetGenerator / NLayerDiscriminator objects: parameters adopted, same
-    state_dict keys, and (on the double) the outputs, encoder features and every gradient of the reference modules
-    evaluating themselves in fp32, at the bf16-storage floor."""
-    import copy
-    from oracle import ref_stubs
-    ref_stubs.install()
-    import functools
-    import torch.nn as nn
-    from models.modules.discriminators import NLayerDiscriminator
-    from models.modules.resnet_architecture.resnet_generator import ResnetGenerator
+def test_accelerate_swaps_reference_gan_nets_and_matches_their_forward(golden_dir):
+    """accelerate() on the reference's own ResnetGenerator / NLayerDiscriminator objects (stored module trees,
+    oracle/gen_golden_accelerate.py): parameters adopted, same state_dict keys, and (on the double) the outputs, encoder
+    features and every gradient (sampled) of the reference modules evaluating themselves in fp32, at the bf16-storage
+    floor."""
+    from oracle import gan_oracle as G
+    from oracle import skeleton
+    from oracle.gen_golden_accelerate import sample
     import joligen_b200
     from joligen_b200 import nets_gan
-    from oracle import gan_oracle as G
-    norm = functools.partial(nn.InstanceNorm2d, affine=False, track_running_stats=False)
-    cases = ((ResnetGenerator(3, 3, 16, norm_layer=norm, use_dropout=False, n_blocks=2), nets_gan.ResnetGenerator,
-              G.resnet_param_shapes(3, 3, 16, 2), G.resnet_generator, (2,)),
-             (NLayerDiscriminator(3, 16, n_layers=3, norm_layer=norm), nets_gan.NLayerDiscriminator,
-              G.nlayer_d_param_shapes(3, 16, 3), G.nlayer_discriminator, (3,)))
-    for ref, kind, shapes, oracle_fn, oargs in cases:
+    cases = (("resnet", nets_gan.ResnetGenerator, G.resnet_param_shapes(3, 3, 16, 2), G.resnet_generator, (2,)),
+             ("nlayerd", nets_gan.NLayerDiscriminator, G.nlayer_d_param_shapes(3, 16, 3), G.nlayer_discriminator, (3,)))
+    for name, kind, shapes, oracle_fn, oargs in cases:
+        gold = skeleton.load(os.path.join(golden_dir, "accel_gan_%s.pt" % name))
+        ref = gold["module"]
         ref.load_state_dict(G.init_from_shapes(shapes, 77))
-        keep = copy.deepcopy(ref)
         params, keys = dict(ref.named_parameters()), list(ref.state_dict().keys())
         fast = joligen_b200.accelerate(ref)
         assert isinstance(fast, kind) and list(fast.state_dict().keys()) == keys
         assert all(p is params[k] for k, p in fast.named_parameters())
         x = torch.randn(2, 3, 64, 64, generator=torch.Generator().manual_seed(1))
-        yr = keep(x)
-        dy = torch.randn(yr.shape, generator=torch.Generator().manual_seed(2))
-        yr.backward(dy)
+        dy = torch.randn(gold["y"].shape, generator=torch.Generator().manual_seed(2))
         with KD.installed():
             yf = fast(x)
-            assert tuple(yf.shape) == tuple(yr.shape) and rel_l2(yf, yr) < 3e-2
+            assert tuple(yf.shape) == tuple(gold["y"].shape) and rel_l2(yf, gold["y"]) < 3e-2
             yf.backward(dy)
             if kind is nets_gan.ResnetGenerator:
                 ff = fast.get_feats(x, [0, 4, 8, 11])
-                for a, b in zip(ff, keep.get_feats(x, [0, 4, 8, 11])):
-                    assert tuple(a.shape) == tuple(b.shape) and rel_l2(a, b) < 3e-2
+                for a, (shape, b) in zip(ff, gold["feats"]):
+                    assert tuple(a.shape) == shape and rel_l2(sample(a), b) < 3e-2
         emu = _emulated_grads(oracle_fn, shapes, 77, x, dy, *oargs)
-        _check_grads_at_bf16_floor([(k, p.grad) for k, p in fast.named_parameters()],
-                                   {k: p.grad for k, p in keep.named_parameters()}, emu)
+        _check_grads_at_bf16_floor([(k, sample(p.grad)) for k, p in fast.named_parameters()], gold["grads"],
+                                   {k: sample(g) for k, g in emu.items()})
     # variants the mirrors do not implement are refused, not swapped silently
-    with pytest.raises((NotImplementedError, RuntimeError)):
-        joligen_b200.accelerate(ResnetGenerator(3, 3, 16, norm_layer=nn.BatchNorm2d, n_blocks=2))
-    with pytest.raises((NotImplementedError, RuntimeError)):
-        joligen_b200.accelerate(ResnetGenerator(3, 3, 16, norm_layer=norm, n_blocks=2, mobile=True))
-    with pytest.raises((NotImplementedError, RuntimeError)):
-        joligen_b200.accelerate(NLayerDiscriminator(3, 16, n_layers=3, norm_layer=norm, use_dropout=True))
+    for ref in skeleton.load(os.path.join(golden_dir, "accel_gan_refused.pt")):
+        with pytest.raises((NotImplementedError, RuntimeError)):
+            joligen_b200.accelerate(ref)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+
+@pytest.mark.skipif(not ref_stubs.available(), reason=REF_MISSING)
 @pytest.mark.parametrize("nce", [None, "patchnce"])
 def test_reference_cut_model_trains_with_accelerated_nets(golden_dir, nce):
     """The reference's cut_model (example_gan_horse2zebra.json, reduced) through its own optimize_parameters() — GAN +
@@ -405,46 +397,35 @@ _VARIANT_BASE = dict(image_size=32, inner_channel=32, channel_mults=(1, 2), res_
                      num_head_channels=16)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
 @pytest.mark.parametrize("variant", [dict(efficient=True), dict(use_scale_shift_norm=False)])
-def test_unet_variants_oracle_host_stack_and_reference_agree(variant):
-    from oracle import ref_stubs
-    ref_stubs.install()
+def test_unet_variants_oracle_host_stack_and_reference_agree(variant, golden_dir):
+    """The reference generator of each variant (stored module tree and its fp32 forward / gradients,
+    oracle/gen_golden_accelerate.py) vs the oracle, and accelerate() of it on the double."""
     from oracle import palette_oracle as O
-    from models.modules.diffusion_generator import DiffusionGenerator
-    from models.modules.palette_denoise_fn import PaletteDenoiseFn
-    from models.modules.unet_generator_attn.unet_generator_attn import UNet
+    from oracle import skeleton
+    from oracle.gen_golden_accelerate import UNET_VARIANT_BASE, sample
     import joligen_b200
-    cfg = O.UNetCfg(**_VARIANT_BASE, **variant)
+    cfg = O.UNetCfg(**UNET_VARIANT_BASE, **variant)
     params = O.init_params(cfg, 5)
-    unet = UNet(image_size=cfg.image_size, in_channel=cfg.in_channel, inner_channel=cfg.inner_channel,
-                out_channel=cfg.out_channel, res_blocks=list(cfg.res_blocks), attn_res=list(cfg.attn_res), tanh=False,
-                n_timestep_train=cfg.n_timestep_train, n_timestep_test=cfg.n_timestep_test, norm="groupnorm",
-                group_norm_size=cfg.group_norm_size, cond_embed_dim=cfg.cond_embed_dim, channel_mults=cfg.channel_mults,
-                num_heads=cfg.num_heads, num_head_channels=cfg.num_head_channels, efficient=cfg.efficient,
-                use_scale_shift_norm=cfg.use_scale_shift_norm)
-    ref = DiffusionGenerator(denoise_fn=PaletteDenoiseFn(model=unet, cond_embed_dim=cfg.cond_embed_dim, ref_embed_net="",
-                                                         conditioning="", nclasses=2),
-                             sampling_method="ddpm", image_size=cfg.image_size, G_ngf=cfg.inner_channel,
-                             loading_backward_compatibility=False)
+    gold = skeleton.load(os.path.join(golden_dir, "accel_unet_%s.pt" % ("efficient" if cfg.efficient else
+                                                                        "no_scale_shift")))
+    ref = gold["module"]
     assert [(k, tuple(v.shape)) for k, v in ref.named_parameters()] == list(O.generator_param_shapes(cfg).items())
     ref.load_state_dict(params, strict=False)
+    nh_r, ref_grads = gold["noise_hat"], gold["grads"]
     data = O.synthetic_batch(2, cfg.image_size, 9)
     torch.manual_seed(1)
     t, u = O.sample_t_gamma(cfg, 2)
     noise = torch.randn_like(data["gt"])
-    # the reference itself, with the same draws (its forward draws t, u; replay them through the generator's RNG order)
-    torch.manual_seed(1)
-    noise_r, nh_r, _ = ref(data["gt"], data["cond"], data["mask"], None, None, None)
-    assert torch.equal(noise_r, noise)
-    torch.nn.functional.mse_loss(noise_r * data["mask"].clamp(0, 1), nh_r * data["mask"].clamp(0, 1)).backward()
+    # the reference drew the same noise with the same seed (its forward draws t, u, then the noise)
+    assert torch.equal(gold["noise"], noise)
     # (1) the oracle restates the reference (fp32)
     leaves = {k: v.clone().requires_grad_(True) for k, v in params.items()}
     _, nh_o, _ = O.diffusion_forward(leaves, data["gt"], data["cond"], data["mask"], noise, t, u, cfg)
     assert rel_l2(nh_o, nh_r) < 1e-4
     O.palette_loss(noise, nh_o, data["mask"]).backward()
-    for k, p in ref.named_parameters():
-        assert rel_l2(leaves[k].grad, p.grad) < 1e-3 or float(p.grad.norm()) < 1e-6, k
+    for k in ref_grads:
+        assert rel_l2(sample(leaves[k].grad), ref_grads[k]) < 1e-3 or float(ref_grads[k].norm()) < 1e-6, k
     # (2) the accelerated reference net on the double, seeded the same way, at the bf16 floor of THIS net (measured: the
     # oracle with the CUDA path's rounding points vs fp32; the 1/sqrt(2) skip weight makes the efficient variant noisier)
     emu = {k: v.clone().requires_grad_(True) for k, v in params.items()}
@@ -456,12 +437,11 @@ def test_unet_variants_oracle_host_stack_and_reference_agree(variant):
         O.EMULATE_BF16[0] = False
     floor = rel_l2(nh_e, nh_r)
     gerr = gnrm = 0.0
-    for k, q in ref.named_parameters():
-        gerr += float((emu[k].grad.double() - q.grad.double()).norm()) ** 2
-        gnrm += float(q.grad.double().norm()) ** 2
+    for k, q in ref_grads.items():
+        gerr += float((sample(emu[k].grad).double() - q.double()).norm()) ** 2
+        gnrm += float(q.double().norm()) ** 2
     gfloor = (gerr / gnrm) ** 0.5
-    import copy
-    fast = joligen_b200.accelerate(copy.deepcopy(ref))
+    fast = joligen_b200.accelerate(ref)
     fast.zero_grad()
     with KD.installed():
         torch.manual_seed(1)
@@ -469,44 +449,35 @@ def test_unet_variants_oracle_host_stack_and_reference_agree(variant):
         assert torch.equal(noise_f, noise) and rel_l2(nh_f, nh_r) < max(3e-2, 1.5 * floor), (rel_l2(nh_f, nh_r), floor)
         torch.nn.functional.mse_loss(noise_f * data["mask"].clamp(0, 1), nh_f * data["mask"].clamp(0, 1)).backward()
     err = nrm = 0.0
-    for (k, p), (_, q) in zip(fast.named_parameters(), ref.named_parameters()):
-        err += float((p.grad.double() - q.grad.double()).norm()) ** 2
-        nrm += float(q.grad.double().norm()) ** 2
+    for k, p in fast.named_parameters():
+        q = ref_grads[k]
+        err += float((sample(p.grad).double() - q.double()).norm()) ** 2
+        nrm += float(q.double().norm()) ** 2
     assert (err / nrm) ** 0.5 < max(4e-2, 1.5 * gfloor), ((err / nrm) ** 0.5, gfloor)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+
 @pytest.mark.parametrize("norm", ["instancenorm", "layernorm", "groupnorm"])
-def test_accelerate_rebuilds_the_reference_norm_variant(norm):
+def test_accelerate_rebuilds_the_reference_norm_variant(norm, golden_dir):
     """--G_unet_mha_norm_layer instancenorm (GroupNorm(C, C): the group count follows each block's width) / layernorm
     (GroupNorm(1, C)) / groupnorm N: accelerate() must rebuild every block's normalisation, not the first block's group
-    count everywhere — checked structurally and against the reference's own forward."""
-    import copy
-    from oracle import ref_stubs
-    ref_stubs.install()
+    count everywhere — checked structurally and against the reference's own forward (stored)."""
+    from oracle import skeleton
     import torch.nn as nn
-    from models.modules.unet_generator_attn.unet_generator_attn import UNet
     import joligen_b200
-    torch.manual_seed(0)
-    ref = UNet(image_size=32, in_channel=6, inner_channel=32, out_channel=3, res_blocks=[1, 1], attn_res=[2], tanh=False,
-               n_timestep_train=2000, n_timestep_test=1000, norm=norm, group_norm_size=8, cond_embed_dim=32,
-               channel_mults=(1, 2), num_heads=1, num_head_channels=16)
-    with torch.no_grad():   # the reference zero-initialises the second conv of every block: de-zero for a real check
-        for p in ref.parameters():
-            if float(p.abs().max()) == 0.0:
-                p.normal_(0.0, 0.05)
-    fast = joligen_b200.accelerate(copy.deepcopy(ref))
+    gold = skeleton.load(os.path.join(golden_dir, "accel_norm_%s.pt" % norm))
+    ref = skeleton.seed_(gold["module"], 3)
     groups = lambda m: [(g.num_groups, g.num_channels) for g in m.modules() if isinstance(g, nn.GroupNorm)]  # noqa: E731
-    assert groups(fast) == groups(ref)
-    x = torch.randn(2, 6, 32, 32)
-    emb = torch.randn(2, 32)
-    want = ref(x, emb)
+    want_groups = groups(ref)
+    fast = joligen_b200.accelerate(ref)
+    assert groups(fast) == want_groups
     with KD.installed():
-        got = fast(x, emb)
-    assert rel_l2(got, want) < 4e-2, rel_l2(got, want)
+        got = fast(gold["x"], gold["emb"])
+    assert rel_l2(got, gold["y"]) < 4e-2, rel_l2(got, gold["y"])
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+
+@pytest.mark.skipif(not ref_stubs.available(), reason=REF_MISSING)
 def test_reference_palette_inference_with_accelerated_generator():
     """PaletteModel.inference (palette_model.py:622-760: set_new_noise_schedule on the denoiser, set_new_sampling_method,
     netG.restoration(y_cond=, y_t=, y_0=, mask=, sample_num=, cls=, ddim_num_steps=, ddim_eta=)) on the accelerated
@@ -535,7 +506,7 @@ def test_reference_palette_inference_with_accelerated_generator():
     assert rel_l2(outs[1][0], outs[0][0]) < 3e-2 and rel_l2(outs[1][1], outs[0][1]) < 3e-2
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not ref_stubs.available(), reason=REF_MISSING)
 def test_reference_checkpoints_interchange_with_accelerated_nets():
     """BaseModel.save_networks / load_networks (base_model.py:824-868, 957-1103) on a model whose netG_A was accelerated:
     the files load into an UNMODIFIED reference net (all keys matched), and into another accelerated model — whose
@@ -576,7 +547,7 @@ def test_reference_checkpoints_interchange_with_accelerated_nets():
         assert rel_l2(want, plain.netG_A.denoise_fn.model(x, emb)) < 3e-2
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not ref_stubs.available(), reason=REF_MISSING)
 def test_train_launcher_hook_accelerates_the_models_train_py_creates():
     """joligen_b200.train: the create_model hook (what `python -m joligen_b200.train` installs in every rank) swaps the
     nets of the models joliGEN's own train.py builds — palette_model and cut_model — and leaves the rest alone."""
@@ -606,176 +577,131 @@ def test_train_launcher_hook_accelerates_the_models_train_py_creates():
         ref_train._jg_hooked = False
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
 @pytest.mark.parametrize("padding_type", ["replicate", "zeros"])
-def test_accelerate_resnet_generator_padding_types(padding_type):
+def test_accelerate_resnet_generator_padding_types(padding_type, golden_dir):
     """--G_padding_type replicate / zeros (resnet_generator.py:42-50, 328-336): accelerate() reads it off the layers,
     the mirror runs nn.ReplicationPad2d through jg_pad2d (mode 1) / the zero padding inside the convolution — output,
-    encoder features and input gradient vs the reference module itself."""
-    import copy
-    import functools
-    from oracle import ref_stubs
-    ref_stubs.install()
-    import torch.nn as nn
-    from models.modules.resnet_architecture.resnet_generator import ResnetGenerator
+    encoder features and input gradient vs the reference module itself (stored)."""
+    from oracle import gan_oracle as G
+    from oracle import skeleton
+    from oracle.gen_golden_accelerate import sample
     import joligen_b200
     from joligen_b200 import nets_gan
-    from oracle import gan_oracle as G
-    norm = functools.partial(nn.InstanceNorm2d, affine=False, track_running_stats=False)
-    ref = ResnetGenerator(3, 3, 16, norm_layer=norm, use_dropout=False, n_blocks=2, padding_type=padding_type)
+    gold = skeleton.load(os.path.join(golden_dir, "accel_resnet_padding_%s.pt" % padding_type))
+    ref = gold["module"]
     seeded = list(G.init_from_shapes(G.resnet_param_shapes(3, 3, 16, 2), 77).values())
     ref.load_state_dict(dict(zip(ref.state_dict().keys(), seeded)))   # (the layer indices shift without pad layers)
-    fast = joligen_b200.accelerate(copy.deepcopy(ref))
+    ref_layers = [type(m).__name__ for m in ref.decoder.model]
+    fast = joligen_b200.accelerate(ref)
     assert isinstance(fast, nets_gan.ResnetGenerator)
-    assert [type(m).__name__ for m in fast.decoder.model] == [type(m).__name__ for m in ref.decoder.model]
+    assert [type(m).__name__ for m in fast.decoder.model] == ref_layers
     x = torch.randn(2, 3, 64, 64, generator=torch.Generator().manual_seed(1))
-    xr, xf = x.clone().requires_grad_(True), x.clone().requires_grad_(True)
-    yr = ref(xr)
-    dy = torch.randn(yr.shape, generator=torch.Generator().manual_seed(2))
-    yr.backward(dy)
+    xf = x.clone().requires_grad_(True)
+    dy = torch.randn(gold["y"].shape, generator=torch.Generator().manual_seed(2))
     with KD.installed():
         yf = fast(xf)
-        assert rel_l2(yf, yr) < 3e-2
+        assert rel_l2(yf, gold["y"]) < 3e-2
         yf.backward(dy)
-        for a, b in zip(fast.get_feats(x, [0, 4, 8, 11]), ref.get_feats(x, [0, 4, 8, 11])):
-            assert tuple(a.shape) == tuple(b.shape) and rel_l2(a, b) < 3e-2
-    assert rel_l2(xf.grad, xr.grad) < 0.3   # (InstanceNorm backward under bf16 storage: see the floor tests above)
+        for a, (shape, b) in zip(fast.get_feats(x, [0, 4, 8, 11]), gold["feats"]):
+            assert tuple(a.shape) == shape and rel_l2(sample(a), b) < 3e-2
+    assert rel_l2(xf.grad, gold["x_grad"]) < 0.3   # (InstanceNorm backward under bf16 storage: see the floor tests above)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
-def test_accelerate_wavelet_space_unet_vs_reference():
+
+def test_accelerate_wavelet_space_unet_vs_reference(golden_dir):
     """--train_feat_wavelet (UNet(freq_space=True), unet_generator_attn.py:467-473, 69-96, 113-140): the net works on
     the Haar bands of its input / output and resamples in pixel space (inverse transform -> resample -> transform).
     The mirror composes jg_haar with the layout / resample kernels; accelerate() adopts the filter buffers — output and
-    input gradient vs the reference's own forward / backward."""
-    import copy
-    from oracle import ref_stubs
-    ref_stubs.install()
-    from models.modules.unet_generator_attn.unet_generator_attn import UNet
+    input gradient vs the reference's own forward / backward (stored)."""
+    from oracle import skeleton
     import joligen_b200
     from joligen_b200 import nets
-    torch.manual_seed(0)
-    ref = UNet(image_size=32, in_channel=6, inner_channel=32, out_channel=3, res_blocks=[1, 1], attn_res=[2], tanh=False,
-               n_timestep_train=2000, n_timestep_test=1000, norm="groupnorm", group_norm_size=8, cond_embed_dim=32,
-               channel_mults=(1, 2), num_heads=1, num_head_channels=16, freq_space=True)
-    with torch.no_grad():
-        for p in ref.parameters():
-            if float(p.abs().max()) == 0.0:
-                p.normal_(0.0, 0.05)
+    gold = skeleton.load(os.path.join(golden_dir, "accel_wavelet_unet.pt"))
+    ref = skeleton.seed_(gold["module"], 3)
     keys = list(ref.state_dict().keys())
-    fast = joligen_b200.accelerate(copy.deepcopy(ref))
+    fast = joligen_b200.accelerate(ref)
     assert isinstance(fast, nets.UNet) and fast.freq_space and list(fast.state_dict().keys()) == keys
-    assert (fast.in_channel, fast.out_channel) == (ref.in_channel, ref.out_channel) == (6, 3)
-    x = torch.randn(1, 6, 32, 32)
-    emb = torch.randn(1, 32)
-    xr, xf = x.clone().requires_grad_(True), x.clone().requires_grad_(True)
-    want = ref(xr, emb)
-    dy = torch.randn_like(want)
-    want.backward(dy)
+    assert (fast.in_channel, fast.out_channel) == (6, 3)
+    xf = gold["x"].clone().requires_grad_(True)
+    want = gold["y"]
     with KD.installed():
-        got = fast(xf, emb)
+        got = fast(xf, gold["emb"])
         assert tuple(got.shape) == tuple(want.shape) == (1, 3, 32, 32)
         assert rel_l2(got, want) < 4e-2, rel_l2(got, want)
-        got.backward(dy)
-    assert rel_l2(xf.grad, xr.grad) < 0.1, rel_l2(xf.grad, xr.grad)
+        got.backward(gold["dy"])
+    assert rel_l2(xf.grad, gold["x_grad"]) < 0.1, rel_l2(xf.grad, gold["x_grad"])
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
-def test_accelerate_wavelet_space_discriminator_vs_reference():
+
+def test_accelerate_wavelet_space_discriminator_vs_reference(golden_dir):
     """NLayerDiscriminator(freq_space=True) (discriminators.py:40-46, 112-117): the PatchGAN reads the Haar bands."""
-    import copy
-    import functools
-    from oracle import ref_stubs
-    ref_stubs.install()
-    import torch.nn as nn
-    from models.modules.discriminators import NLayerDiscriminator
+    from oracle import skeleton
     import joligen_b200
-    from joligen_b200 import nets_gan
-    norm = functools.partial(nn.InstanceNorm2d, affine=False, track_running_stats=False)
-    torch.manual_seed(1)
-    ref = NLayerDiscriminator(3, 16, n_layers=3, norm_layer=norm, freq_space=True)
+    from joligen_b200 import nets_gan, ops
+    gold = skeleton.load(os.path.join(golden_dir, "accel_wavelet_nlayerd.pt"))
+    ref = skeleton.seed_(gold["module"], 4)
     keys = list(ref.state_dict().keys())
-    fast = joligen_b200.accelerate(copy.deepcopy(ref))
+    fast = joligen_b200.accelerate(ref)
     assert isinstance(fast, nets_gan.NLayerDiscriminator) and fast.freq_space and list(fast.state_dict().keys()) == keys
-    x = torch.randn(2, 3, 128, 128)
-    want = ref(x)
+    x, want = gold["x"], gold["y"]
     with KD.installed():
         got = fast(x)
-        from joligen_b200 import ops
         got2 = ops.to_nchw(fast.forward_nhwc(ops.to_nhwc(x)), 1)     # the trainers' NHWC entry point
     assert tuple(got.shape) == tuple(want.shape) and rel_l2(got, want) < 3e-2 and rel_l2(got2, want) < 3e-2
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
-def test_accelerate_spectral_norm_discriminator_vs_reference():
+
+def test_accelerate_spectral_norm_discriminator_vs_reference(golden_dir):
     """--D_spectral: NLayerDiscriminator of torch-spectral_norm-wrapped convolutions (`weight_orig`, `weight_u`,
     `weight_v` in the state_dict).  The wrapper's pre-forward hook never runs on the B200 path: the mirror does the power
-    iteration and the normalisation itself (nets_projd._sn_weight) — logits, every gradient and the u / v buffers after
-    one training-mode forward vs the reference module."""
-    import copy
-    import functools
-    from oracle import ref_stubs
-    ref_stubs.install()
-    import torch.nn as nn
-    from models.modules.discriminators import NLayerDiscriminator
+    iteration and the normalisation itself (nets_projd._sn_weight) — logits, the last layer's gradient and the u / v
+    buffers after one training-mode forward vs the reference module (stored)."""
+    from oracle import skeleton
+    from oracle.gen_golden_accelerate import sample
     import joligen_b200
     from joligen_b200 import nets_gan
-    norm = functools.partial(nn.InstanceNorm2d, affine=False, track_running_stats=False)
-    torch.manual_seed(2)
-    ref = NLayerDiscriminator(3, 16, n_layers=3, norm_layer=norm, use_spectral=True).train()
+    gold = skeleton.load(os.path.join(golden_dir, "accel_spectral_nlayerd.pt"))
+    ref = skeleton.seed_(gold["module"], 2).train()
     keys = list(ref.state_dict().keys())
-    fast = joligen_b200.accelerate(copy.deepcopy(ref))
+    fast = joligen_b200.accelerate(ref)
     assert isinstance(fast, nets_gan.NLayerDiscriminator) and list(fast.state_dict().keys()) == keys
     assert any(k.endswith("weight_orig") for k in keys) and any(k.endswith("weight_u") for k in keys)
-    x = torch.randn(2, 3, 96, 96)
-    want = ref(x)
-    dy = torch.randn_like(want)
-    want.backward(dy)
     with KD.installed():
-        got = fast(x)
-        assert rel_l2(got, want) < 3e-2, rel_l2(got, want)
-        got.backward(dy)
-    for (k, a), (_, b) in zip(fast.state_dict().items(), ref.state_dict().items()):
-        if k.endswith(("weight_u", "weight_v")):   # the power iteration is fp32 torch arithmetic on both sides
-            assert float((a - b).abs().max()) < 1e-5, k
-    named = dict(ref.named_parameters())
-    last = [k for k in named if k.endswith("weight_orig")][-1]
-    assert rel_l2(dict(fast.named_parameters())[last].grad, named[last].grad) < 3e-2
+        got = fast(gold["x"])
+        assert rel_l2(got, gold["y"]) < 3e-2, rel_l2(got, gold["y"])
+        got.backward(gold["dy"])
+    sd = fast.state_dict()
+    for k, b in gold["uv_after"].items():   # the power iteration is fp32 torch arithmetic on both sides
+        assert float((sd[k] - b).abs().max()) < 1e-5, k
+    last = [k for k in keys if k.endswith("weight_orig")][-1]
+    assert rel_l2(sample(dict(fast.named_parameters())[last].grad), gold["grads"][last]) < 3e-2
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
-def test_accelerate_spectral_norm_generator_vs_reference():
+
+def test_accelerate_spectral_norm_generator_vs_reference(golden_dir):
     """--G_spectral: ResnetGenerator whose convolutions AND transposed convolutions are spectral_norm-wrapped (the matrix
     rows of a ConvTranspose2d are its OUTPUT channels: dim 1) — output, the u / v buffers after one training-mode
-    forward and the gradient of a transposed-convolution weight vs the reference module."""
-    import copy
-    import functools
-    from oracle import ref_stubs
-    ref_stubs.install()
-    import torch.nn as nn
-    from models.modules.resnet_architecture.resnet_generator import ResnetGenerator
+    forward and the gradient of a transposed-convolution weight vs the reference module (stored)."""
+    from oracle import skeleton
+    from oracle.gen_golden_accelerate import sample
     import joligen_b200
     from joligen_b200 import nets_gan
-    norm = functools.partial(nn.InstanceNorm2d, affine=False, track_running_stats=False)
-    torch.manual_seed(4)
-    ref = ResnetGenerator(3, 3, 16, norm_layer=norm, use_dropout=False, n_blocks=2, use_spectral=True).train()
+    gold = skeleton.load(os.path.join(golden_dir, "accel_spectral_resnet.pt"))
+    ref = skeleton.seed_(gold["module"], 4).train()
     keys = list(ref.state_dict().keys())
-    fast = joligen_b200.accelerate(copy.deepcopy(ref))
+    fast = joligen_b200.accelerate(ref)
     assert isinstance(fast, nets_gan.ResnetGenerator) and list(fast.state_dict().keys()) == keys
     # wrapped: stem, down- and up-sampling layers; NOT wrapped: the ResnetBlocks (a reference quirk) and the 7x7 head
     assert "decoder.model.0.weight_orig" in keys and "decoder.model.7.weight" in keys
     assert "encoder.model.10.conv_block.1.weight" in keys
-    x = torch.randn(2, 3, 64, 64)
-    want = ref(x)
-    dy = torch.randn_like(want)
-    want.backward(dy)
     with KD.installed():
-        got = fast(x)
-        assert rel_l2(got, want) < 3e-2, rel_l2(got, want)
-        got.backward(dy)
-    for (k, a), (_, b) in zip(fast.state_dict().items(), ref.state_dict().items()):
-        if k.endswith(("weight_u", "weight_v")):
-            assert float((a - b).abs().max()) < 1e-5, k
-    gf = dict(fast.named_parameters())["decoder.model.3.weight_orig"].grad
-    gr = dict(ref.named_parameters())["decoder.model.3.weight_orig"].grad
+        got = fast(gold["x"])
+        assert rel_l2(got, gold["y"]) < 3e-2, rel_l2(got, gold["y"])
+        got.backward(gold["dy"])
+    sd = fast.state_dict()
+    for k, b in gold["uv_after"].items():
+        assert float((sd[k] - b).abs().max()) < 1e-5, k
+    gf = sample(dict(fast.named_parameters())["decoder.model.3.weight_orig"].grad)
+    gr = gold["grads"]["decoder.model.3.weight_orig"]
     assert rel_l2(gf, gr) < 0.15, rel_l2(gf, gr)
+

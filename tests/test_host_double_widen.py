@@ -9,6 +9,10 @@ import torch
 
 import kernel_double as KD
 
+from oracle import ref_stubs  # noqa: E402
+
+REF_MISSING = "needs the reference's own code: build() stages it under oracle/_ref where the checkout is readable"
+
 
 def rel_l2(a, b):
     a, b = a.detach().double(), b.detach().double()
@@ -177,7 +181,7 @@ def test_video_unet_on_the_double(golden_dir):
     _check_unet_grads(dict(net.named_parameters()), leaves, gold)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not ref_stubs.available(), reason=REF_MISSING)
 @pytest.mark.parametrize("which", ["ref", "vid"])
 def test_reference_palette_model_cfg4_cfg5_trains_with_accelerated_generator(golden_dir, which):
     """The unmodified reference's control path for BASELINE config 4 (unet_mha_ref_attn with ref_A) and config 5
@@ -212,7 +216,7 @@ def test_reference_palette_model_cfg4_cfg5_trains_with_accelerated_generator(gol
         assert abs(float(ema[k].double().norm()) - n) <= 2e-2 * n + 1e-6, k
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not ref_stubs.available(), reason=REF_MISSING)
 @pytest.mark.parametrize("which", ["ref", "vid"])
 def test_reference_inference_cfg4_cfg5_with_accelerated_generator(which):
     """PaletteModel.inference for the reference-image UNet (its `use_ref` branch: restoration(..., ref=cur_ref)) and for
@@ -242,7 +246,7 @@ def test_reference_inference_cfg4_cfg5_with_accelerated_generator(which):
     assert rel_l2(outs[1], outs[0]) < 3e-2, rel_l2(outs[1], outs[0])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not ref_stubs.available(), reason=REF_MISSING)
 @pytest.mark.parametrize("cond", ["class", "class_mask"])
 def test_reference_palette_model_with_conditioning_trains_with_accelerated_generator(cond):
     """--alg_diffusion_cond_embed class / class_mask (example_ddpm_mario.json ships `class`) through the reference's own
